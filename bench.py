@@ -5,6 +5,7 @@ include/powdr_b200.h.
 
   python bench.py --gpus N --steps K --warmup W                 # native CUDA arm (torchrun launches N ranks for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W  # the CPU implementation on the host cores (rank 0 only)
+  python bench.py ... --dump-outputs DIR                          # also write the last timed step's proof and openings as DIR/*.npy
 
 One step = one segment per GPU through the whole path: main trace commit (LDE + Poseidon2 Merkle) -> LogUp permutation trace
 (generate, LDE, commit) -> quotient -> quotient commit -> openings at zeta / zeta*w -> FRI commit phase -> proof of work (16 bits)
@@ -53,7 +54,36 @@ def parse():
                     help="keccak: one APC chip per segment (the BASELINE metric); multichip: 50 independent chips of one segment "
                          "sharded over the ranks by LPT (BASELINE.json configs[3] shape, strong scaling); pairing: ONE wide segment "
                          "(default 2^20 x 16384, BASELINE.json configs[4]) column-sharded over all ranks -- the case that needs sharding")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (proof fields, query openings, opened values) as "
+                         "DIR/<name>.npy in float64, so that two builds can be compared output for output (keccak workload, native arm)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "native" or a.workload != "keccak"):
+        ap.error("--dump-outputs is implemented for the keccak workload of the native arm")
+    return a
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, proof, arrays):
+    """proof dict + named arrays -> path/<name>.npy, float64 (every value is a field element or a 32-bit word: exact).  Over
+    DUMP_LIMIT_BYTES in all, a fixed seeded sample of the query rows is kept, with their indices in query_rows.npy."""
+    import numpy as np
+    out = {k: np.asarray(v, dtype=np.float64) for k, v in proof.items()}
+    out.update({k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()})
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        q = out["queries"]
+        keep = (DUMP_LIMIT_BYTES - (total - q.nbytes)) // (8 * (q.shape[1] + 1))      # a row and its index
+        assert keep > 0, "outputs other than the query rows exceed %d bytes" % DUMP_LIMIT_BYTES
+        rows = np.sort(np.random.default_rng(0).choice(q.shape[0], keep, replace=False))
+        out["queries"], out["query_rows"] = q[rows], rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def workload_name(a):
@@ -254,11 +284,11 @@ def run_native(a):
 
     def step_device():
         proof = ctx.prove_segment(air, trace.data_ptr(), a.log_n, w, on_device=True)
-        ctx.query_segment(a.log_n, w, wp)                     # query phase: 100 openings gathered on the device, read back
+        queries, ys = ctx.query_segment(a.log_n, w, wp)      # query phase: 100 openings gathered on the device, read back
         if world > 1:   # the path's one exchange: all-gather of the segment commitments (Merkle caps) over NCCL/NVLink
             caps.copy_(torch.tensor(proof["trace_root"] + proof["quotient_root"], dtype=torch.int64).to(torch.int32), non_blocking=True)
             parallel.all_gather_caps(caps.view(2, 8), dist)
-        return proof
+        return proof, queries, ys
 
     def sync_all():
         torch.cuda.synchronize()
@@ -279,7 +309,7 @@ def run_native(a):
     sampler.mark()
     e0.record(stream)
     for _ in range(a.steps):
-        proof = step_device()
+        proof, queries, ys = step_device()
     e1.record(stream)
     sync_all()
     ms = e0.elapsed_time(e1)
@@ -322,11 +352,14 @@ def run_native(a):
                "d2h_bytes_per_step": (C_sizeof_proof + int(q2.nbytes) + int(ys2.nbytes)) * world,
                "stages_ms": ctx.last_stage_ms()}
 
+    last = (proof, {"queries": queries, "opened_values": ys})
     sharded = None
     if world > 1 and not a.no_sharded:
-        sharded = sharded_segment(a, ctx, air, dist, dev, stream, world, rank)
+        sharded, last = sharded_segment(a, ctx, air, dist, dev, stream, world, rank)
 
     if rank == 0:
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, *last)
         peaks = {}
         try:
             peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -400,7 +433,7 @@ def sharded_segment(a, ctx, air, dist, dev, stream, world, rank):
     """Strong scaling of ONE segment: the N ranks prove the same segment together (pb_prove_segment_sharded: column-sharded
     trace in, one all-to-all of folded coefficients, row-sharded LDE / Merkle / quotient / FRI; NCCL through
     powdr_b200.sharded.TorchComm).  Reported next to the weak-scaling headline; the proof is checked against the
-    single-GPU proof of the same trace on every rank."""
+    single-GPU proof of the same trace on every rank.  -> (result dict, (proof, query openings) of the last device-input step)"""
     import torch
     from powdr_b200.sharded import TorchComm, shard_columns
     n, w = 1 << a.log_n, air.width
@@ -482,7 +515,7 @@ def sharded_segment(a, ctx, air, dist, dev, stream, world, rank):
         out["e2e"] = {"value": esec, "unit": "s", "h2d_bytes_per_step": 4 * w * n, "d2h_bytes_per_step": (ctypes.sizeof(SegmentProof) + (4 * int(single_q.size) if single_q is not None else 0)) * world,
                       "proof_equals_single_gpu": eproof == single,
                       "stages_ms": ctx.last_stage_ms()}
-    return out
+    return out, (proof, {} if queries is None else {"queries": queries})
 
 
 def multichip_shapes():

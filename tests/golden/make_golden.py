@@ -18,6 +18,8 @@ reference-derived fixtures and the oracle for the generated vectors):  python te
                                    single_div_nondet, wasm_register_reuse and keccak_apc_pre_opt (677 instructions, 27 521 cells): the
                                    REAL stage-0 gather pattern (the machines of the big fixture are not committed: 28 627 constraints)
   chips_mixed.json                 three chips of different heights under one transcript (orc_prove_chips): proof, cumulative sums, digests
+  v1_metrics.json                  the OpenVM-1 metrics document powdr_b200.metrics writes for one segment, and the summary the
+                                   reference's own tooling (openvm-riscv/scripts/basic_metrics.py extract_metrics) reads from it
 """
 import glob
 import gzip
@@ -80,6 +82,7 @@ def main():
         with gzip.GzipFile(os.path.join(HERE, "stage0_subs.json.gz"), "wb", mtime=0) as f:
             f.write(json.dumps(st0, separators=(",", ":")).encode())
         print("wrote stage0_subs.json.gz", os.path.getsize(os.path.join(HERE, "stage0_subs.json.gz")), "bytes")
+        v1_metrics()
     rng = np.random.default_rng(2024)
     kat = {}
     kat["perm_zero"] = orc.poseidon2_permute(np.zeros(16, dtype=np.uint32)).tolist()
@@ -125,6 +128,34 @@ def main():
     proof, cs, ys, q = orc.prove_chips(chips, n_queries=g["n_queries"], pow_bits=g["pow_bits"])
     g.update(proof=proof, cumsums=cs.tolist(), ys_sha256=sha(ys), queries_sha256=sha(q))
     dump("chips_mixed.json", g)
+
+
+def v1_metrics():
+    """one segment's stage times through powdr_b200.metrics, then through the reference's basic_metrics.extract_metrics (its
+    matplotlib import serves the plots only and is stubbed where matplotlib is not installed)"""
+    import tempfile
+    import types
+    from powdr_b200 import metrics
+    inputs = {"stage_ms": {"h2d": 0.1, "lde": 34.0, "merkle": 130.0, "logup_gen": 46.0, "logup_commit": 270.0, "quotient": 60.0, "qlde": 0.3,
+                           "qmerkle": 1.3, "open": 25.0, "fri": 3.9, "pow": 0.3, "total": 571.0},
+              "rows": 1 << 20, "main_cols": 2022, "perm_cols": 3348, "n_constraints": 187, "n_interactions": 1734, "trace_gen_ms": 12.0, "query_ms": 0.5}
+    doc = metrics.segment_metrics(inputs["stage_ms"], inputs["rows"], inputs["main_cols"], inputs["perm_cols"], inputs["n_constraints"],
+                                  inputs["n_interactions"], trace_gen_ms=inputs["trace_gen_ms"], query_ms=inputs["query_ms"])
+    try:
+        import matplotlib  # noqa: F401
+    except ImportError:
+        mpl = types.ModuleType("matplotlib")
+        mpl.pyplot, mpl.ticker = types.ModuleType("matplotlib.pyplot"), types.ModuleType("matplotlib.ticker")
+        mpl.ticker.AutoMinorLocator = None
+        sys.modules.update({"matplotlib": mpl, "matplotlib.pyplot": mpl.pyplot, "matplotlib.ticker": mpl.ticker})
+    sys.path.insert(0, os.path.join(REF, "openvm-riscv/scripts"))
+    import basic_metrics
+    with tempfile.TemporaryDirectory() as d:
+        path = os.path.join(d, "metrics.json")
+        metrics.write(path, doc)
+        out = basic_metrics.extract_metrics(path)
+    summary = {k: (float(v) if isinstance(v, float) else int(v)) for k, v in out.items() if k != "filename"}
+    dump("v1_metrics.json", {"inputs": inputs, "metrics": doc, "basic_metrics": summary})
 
 
 def chips_for(spec, seed):

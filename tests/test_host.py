@@ -324,14 +324,15 @@ def test_entry_points_reject_null_arguments_before_touching_the_device():
 
 
 def test_v1_metrics_json_is_consumed_by_the_reference_tooling(tmp_path):
-    """SURVEY §8 f4: the per-stage times go out under the OpenVM-1 metric names; the reference's own basic_metrics.py must be able to
-    read the file (run only where /root/reference exists: the GPU box has no copy)"""
+    """SURVEY §8 f4: the per-stage times go out under the OpenVM-1 metric names.  tests/golden/v1_metrics.json holds the document
+    written for these stage times and the summary the reference's own basic_metrics.extract_metrics read from it
+    (tests/golden/make_golden.py); the writer must still produce that document, byte for byte after parsing"""
     import json
-    import sys
     from powdr_b200 import metrics
-    stage = {"h2d": 0.1, "lde": 34.0, "merkle": 130.0, "logup_gen": 46.0, "logup_commit": 270.0, "quotient": 60.0, "qlde": 0.3, "qmerkle": 1.3,
-             "open": 25.0, "fri": 3.9, "pow": 0.3, "total": 571.0}
-    m = metrics.segment_metrics(stage, 1 << 20, 2022, 3348, 187, 1734, trace_gen_ms=12.0, query_ms=0.5)
+    gold = json.load(open(os.path.join(GOLDEN, "v1_metrics.json")))
+    inp = gold["inputs"]
+    m = metrics.segment_metrics(inp["stage_ms"], inp["rows"], inp["main_cols"], inp["perm_cols"], inp["n_constraints"], inp["n_interactions"],
+                                trace_gen_ms=inp["trace_gen_ms"], query_ms=inp["query_ms"])
     path = tmp_path / "metrics.json"
     metrics.write(str(path), m)
     doc = json.load(open(path))
@@ -339,21 +340,8 @@ def test_v1_metrics_json_is_consumed_by_the_reference_tooling(tmp_path):
     for k in ("main_trace_commit_time_ms", "perm_trace_commit_time_ms", "quotient_poly_compute_time_ms", "quotient_poly_commit_time_ms",
               "pcs_opening_time_ms", "stark_prove_excluding_trace_time_ms", "total_proof_time_ms", "trace_gen_time_ms"):
         assert k in names
-    scripts = "/root/reference/openvm-riscv/scripts"
-    if not os.path.isdir(scripts):
-        return
-    sys.path.insert(0, scripts)
-    try:
-        import matplotlib                      # noqa: F401  (basic_metrics imports it at module level)
-        import basic_metrics
-    except Exception:
-        import metrics_utils
-        app, leaf, internal = metrics_utils.load_metrics_dataframes(str(path))
-        assert len(app) > 0
-        return
-    finally:
-        sys.path.remove(scripts)
-    out = basic_metrics.extract_metrics(str(path))
+    assert doc == gold["metrics"]
+    out = gold["basic_metrics"]
     assert out["num_segments"] == 1 and out["powdr_ratio"] == 1.0 and out["powdr_rows"] == 1 << 20
     assert abs(out["app_proof_time_excluding_trace_ms"] - 571.5) < 1e-6 and out["app_proof_cols"] == 2022 + 3348
 
@@ -394,3 +382,25 @@ def test_host_transcript_generic_diagonal_branch(tmp_path):
                            os.path.join(ROOT, "powdr_b200", "csrc", "transcript_host.cpp")])
     r = subprocess.run([exe], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0 and "bad=0" in r.stdout, r.stdout + r.stderr
+
+
+def test_bench_dump_outputs_is_exact_and_capped(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: field elements and 32-bit words survive the float64 files exactly; above the size cap a fixed,
+    seeded sample of the query rows is written together with its row indices"""
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    proof = {"trace_root": list(range(8)), "fri_roots": [[7] * 8] * 3, "final_poly": [], "pow_witness": 2**32 - 1}
+    q = np.random.default_rng(1).integers(0, 2**32, (100, 500), dtype=np.uint32)
+    ys = np.arange(40, dtype=np.uint32).reshape(10, 4)
+    bench.dump_outputs(str(tmp_path / "all"), proof, {"queries": q, "opened_values": ys})
+    assert (np.load(tmp_path / "all" / "queries.npy") == q).all() and (np.load(tmp_path / "all" / "opened_values.npy") == ys).all()
+    assert np.load(tmp_path / "all" / "pow_witness.npy") == 2**32 - 1 and np.load(tmp_path / "all" / "fri_roots.npy").shape == (3, 8)
+    assert not (tmp_path / "all" / "query_rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 1 << 17)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), proof, {"queries": q, "opened_values": ys})
+        assert sum(f.stat().st_size - 128 for f in (tmp_path / d).iterdir()) <= 1 << 17        # .npy header: 128 bytes
+    rows = np.load(tmp_path / "s1" / "query_rows.npy").astype(np.int64)
+    assert 0 < len(rows) < 100 and (np.load(tmp_path / "s1" / "queries.npy") == q[rows]).all()
+    assert (rows == np.load(tmp_path / "s2" / "query_rows.npy")).all()
