@@ -3,7 +3,7 @@ primitive it re-implements -- so that timing it (bench.py cpu_baseline / --impl 
 import numpy as np
 import pytest
 
-from util import P, rand_field
+from util import P, rand_field, root_of_unity, structured_columns, lde_mismatch, merkle_mismatch, proof_mismatch
 
 
 @pytest.fixture(scope="module")
@@ -56,3 +56,47 @@ def test_fast_openings_and_reduced_opening(fast):
     other = rand_field(rng, (3, 2 << log_n))
     ys = rand_field(rng, (w + 3, 4))
     assert (fast.fast_deep_quotient([lde, other], 31, zeta, gamma, ys) == fast.deep_quotient([lde, other], 31, zeta, gamma, ys)).all()
+
+
+# ---- the sizes the CPU arm vouches for when the GPU is checked against it (tests/test_gpu_scale_parity.py): past BLK_LOG = 18 in
+# oracle/fast.c, where the cache-blocked NTT stages and the tiled bit reversal take over, and whole proofs at 2^16 ----
+def _w2n_inv(log_n):
+    return pow(root_of_unity(log_n + 1), P - 2, P)
+
+
+@pytest.mark.parametrize("log_n,width,log_blowup,shift", [(19, 8, 1, 31), (19, 7, 1, 1), (19, 7, 1, "w2n_inv"), (19, 7, 2, 31), (20, 8, 1, 31),
+                                                          (20, 7, 1, "w2n_inv"), (21, 7, 1, 31)])
+def test_fast_lde_past_the_blocked_stages(fast, log_n, width, log_blowup, shift):
+    shift = _w2n_inv(log_n) if shift == "w2n_inv" else shift
+    t = structured_columns(np.random.default_rng(1000 + log_n), 1 << log_n, width)
+    got, exp = fast.fast_lde_batch(t, log_blowup, shift), fast.lde_batch(t, log_blowup, shift)
+    assert lde_mismatch(got, exp, t, log_blowup, shift) is None, lde_mismatch(got, exp, t, log_blowup, shift, fast)
+
+
+@pytest.mark.parametrize("widths,log_h", [([4, 4], 17), ([3, 16], 18)])
+def test_fast_merkle_every_layer_at_scale(fast, widths, log_h):
+    rng = np.random.default_rng(log_h)
+    mats = [rand_field(rng, (w, 1 << log_h)) for w in widths]
+    got, exp = fast.fast_merkle_commit(mats), fast.merkle_commit(mats)
+    assert merkle_mismatch(got, exp, mats) is None, merkle_mismatch(got, exp, mats, fast)
+
+
+def test_fast_prove_equals_scalar_prove_at_2p16_with_interactions(fast):
+    """64 columns, 8 constraints, 40 interactions (a quadratic one every 7th): the proof, the opened values and the query openings"""
+    from powdr_b200 import machine as M
+    base = M.synthetic_machine(64, 8, seed=16)
+    mach = M.SymbolicMachine(base.constraints, M.synthetic_bus(base, 40, seed=16, quadratic_every=7))
+    bc, spans = M.compile_constraints(mach)
+    bus = M.compile_bus(mach, 1)
+    trace = rand_field(np.random.default_rng(16), (mach.width, 1 << 16))
+    got, exp = fast.prove(trace, bc, spans, bus, fast=True)[:3], fast.prove(trace, bc, spans, bus)[:3]
+    assert proof_mismatch(got, exp) is None, proof_mismatch(got, exp)
+
+
+def test_fast_prove_chips_equals_scalar_with_a_2p15_chip(fast):
+    from test_oracle_chips import _chips
+    chips = _chips([(15, 24, 3, 12), (13, 40, 0, 20), (11, 9, 4, 0), (13, 16, 2, 6)], seed=15)
+    gp, gcs, gys, gq = fast.prove_chips(chips, fast=True)
+    ep, ecs, eys, eq = fast.prove_chips(chips)
+    assert proof_mismatch((gp, gys, gq), (ep, eys, eq)) is None, proof_mismatch((gp, gys, gq), (ep, eys, eq))
+    assert (gcs == ecs).all()
